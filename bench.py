@@ -27,6 +27,12 @@ states.  Rank 0 prints one JSON line.
 --impl reference times the CPU oracle on the host cores (the reference's own OSQP-based binary cannot be
 built here: no Eigen / OSQP / osqp-eigen / glog / gflags in the image), same `config` object, same JSON
 contract; each step is a bounded sample of the workload (stated in cpu_baseline.sample).
+
+--dump-outputs DIR writes what the timed call returned in its last timed step (rank 0's shard) as float64
+.npy files, so that two builds run with the same arguments can be compared output for output (the inputs
+are seeded): status.npy, iters.npy (per path), paths.npy (the path indices the per-station files cover),
+states.npy (rows x 7: x, y, z, k, s, v, a) and frenet.npy (rows x 3).  The per-station files cover every
+path, or a fixed seeded sample of whole paths where that would exceed 64 MB in all.
 """
 import argparse
 import ctypes as C
@@ -49,6 +55,8 @@ from path_optimizer_b200.abi import BOUNDS_DTYPE, STATE_DTYPE, Stats  # noqa: E4
 METRIC = "path_qp_solves_per_sec"
 UNIT = "solves/s"
 CPU_SAMPLE_PATHS = 1024      # paths per CPU step for configs whose shard is larger than that
+DUMP_LIMIT_BYTES = 64 * 1000 * 1000
+DUMP_SEED = 0
 
 
 def io_bytes_per_solve(n):
@@ -59,6 +67,28 @@ def io_bytes_per_solve(n):
 def w_iter_bytes(n):
     """SURVEY.md 8(d) per-iteration working set W_iter(N) = 236 N floats = 944 N bytes."""
     return 944 * n
+
+
+def dump_outputs(out_dir, n_points, states, frenet, status, iters):
+    """Writes one step's outputs of a batch as float64 .npy files under `out_dir` (see --dump-outputs)."""
+    n_points = np.asarray(n_points, dtype=np.int64)
+    B = len(n_points)
+    off = np.concatenate([[0], np.cumsum(n_points)])
+    row_bytes = (len(STATE_DTYPE.names) + 3) * 8
+    max_rows = (DUMP_LIMIT_BYTES - 3 * 8 * B - 5 * 128) // row_bytes    # 5 files, 128-byte .npy headers
+    if off[-1] <= max_rows:
+        paths = np.arange(B)
+    else:
+        order = np.random.default_rng(DUMP_SEED).permutation(B)
+        paths = np.sort(order[np.cumsum(n_points[order]) <= max_rows])
+    rows = np.concatenate([np.arange(off[p], off[p + 1]) for p in paths])
+    states = np.asarray(states)[rows]
+    out = {"status": status, "iters": iters, "paths": paths,
+           "states": np.stack([states[f] for f in STATE_DTYPE.names], axis=1),
+           "frenet": np.asarray(frenet).reshape(-1, 3)[rows]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(arr, dtype=np.float64))
 
 
 def measured_peak_gbs():
@@ -233,6 +263,8 @@ def run_reference(args, rank, world):
         r = cpu_solve(oracle, params, F, batch, threads)
         step_s.append(r["seconds"])
         solved += int((r["status"] == 1).sum())
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, batch["n_points"], r["states"], r["frenet"], r["status"], r["iters"])
     secs = sum(step_s)
     value = B * args.steps / secs
     line = {
@@ -499,6 +531,10 @@ def run_ours(args, rank, world, local_rank):
         sampler.start()
     r = time_workload(w, torch, args.steps, args.warmup, flush, stream, barrier)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the device buffers still hold the last timed step: the host-buffer arm writes its own pinned buffers
+        dump_outputs(args.dump_outputs, w.h_n, w.d_out.cpu().numpy().view(STATE_DTYPE), w.d_frenet[:w.total * 3].cpu().numpy(),
+                     r["status"], r["iters"])
 
     # ---- reduce over ranks: step time = max over ranks; per-rank breakdown gathered as it is
     t = torch.tensor([r["dev_ms"], r["e2e_ms"], r["wall_ms"]], dtype=torch.float64, device=dev)
@@ -727,7 +763,10 @@ def main():
                     help="type string of OsqpSolver::create to solve the config with (default KP: the BASELINE metric)")
     ap.add_argument("--cpu-threads", type=int, default=0, help="CPU arm thread count (default: physical cores)")
     ap.add_argument("--no-extras", action="store_true", help="skip the config 3/4/5 context measurements of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as .npy files under DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
